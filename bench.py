@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the gradient-inversion hot path (BASELINE.json metric).
 
-    python bench.py --gpus N --steps K --warmup W [--config C]             # product arm: the sm_100a engine
+    python bench.py --gpus N --steps K --warmup W [--config C] [--dump-outputs DIR]   # product arm: the sm_100a engine
     python bench.py --impl reference --steps K --warmup W [--config C]     # reference arm: CPU restatement of the reference loop
 
 A "step" is one iteration of ``OptimizationBasedAttacker._run_trial`` (closure + optimiser step + projection + best-so-far)
@@ -388,6 +388,7 @@ class EngineRunner:
         self.cfg, self.config = cfg, config
         opt = cfg.optim
         table = lr_table(opt.step_size, opt.step_size_decay, opt.warmup, opt.max_iterations)
+        self.history_cap = len(table)  # the engine keeps the objective of the first len(table) iterations
         torch.manual_seed(1000 + rank)  # every rank = an independent restart
         local = shared[0]["metadata"]["local_hyperparams"]
         self.local_steps = 0 if local is None else int(local["steps"])
@@ -432,6 +433,32 @@ class EngineRunner:
 
     def timed(self, n):
         return self.eng.run_timed(n)
+
+    def outputs(self):
+        """What a caller of the trial reads back after the last step: the current and the best-so-far candidate, the objective of
+        every recorded iteration (warm-up and timed) and, for the joint text attack, the current and best label logits."""
+        eng = self.eng
+        recorded = eng.status()["recorded"]
+        out = dict(candidate=eng.candidate(), best=eng.best(), objective_history=eng.history(min(recorded, self.history_cap)))
+        if self.config == 5:
+            out.update(labels=eng.joint_labels(best=False), best_labels=eng.joint_labels(best=True))
+        return out
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(outputs, directory):
+    """Write every output as ``directory/<name>.npy`` (float32).  The largest configuration (5) writes about 13 MB."""
+    import numpy as np
+
+    arrays = {name: t.detach().cpu().numpy().astype(np.float32) for name, t in outputs.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"bench.py: outputs of {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte dump limit")
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 
 def host_payload(case, config):
@@ -490,6 +517,8 @@ def product_arm(args):
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms_max = float(t.item())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(runner.outputs(), args.dump_outputs)
     st = runner.eng.status()
     launches = runner.eng.launches_per_iteration()
     prog, n_params, local_steps = runner.prog, runner.n_params, runner.local_steps
@@ -645,7 +674,11 @@ def main():
     ap.add_argument("--cpu-steps", type=int, default=0)
     ap.add_argument("--eager-steps", type=int, default=200)
     ap.add_argument("--skip-eager", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the trial's outputs (rank 0) as DIR/<name>.npy, to compare two builds")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the product arm")
     if args.impl == "reference":
         args.steps = WORKLOADS[args.config]["ref_steps"] if args.steps is None else args.steps
         args.warmup = 3 if args.warmup is None else args.warmup

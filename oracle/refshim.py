@@ -3,8 +3,8 @@
 TEST INFRASTRUCTURE ONLY.  Works only where ``/root/reference`` exists (the build
 container); the GPU box has no reference tree, so nothing on the ``-m gpu`` path,
 ``smoke()`` or ``bench.py`` touches this module.  It is used by
-``tests/golden/make_golden.py`` to produce the committed fixtures and by the CPU
-tests that pin ``oracle/restate.py`` directly against the live reference.
+``tests/golden/make_golden.py`` to produce the committed fixtures; the tests use
+only its ``RefCfg`` config objects and compare against those fixtures.
 
 Shims (SURVEY.md section 8c):
   * ``hydra`` / ``omegaconf`` are not installed -> stub modules in ``sys.modules``

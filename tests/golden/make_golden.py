@@ -317,7 +317,70 @@ def config_fixtures():
     return {n: plain(refshim.load_reference_attack_cfg(n)) for n in names}
 
 
+def dropin_fixture(ref):
+    """What the drop-in tests compare against: the reference attacker's text prologue / token recovery on the miniature causal-LM
+    case, and the reference's own ``TransformerModel`` (weights, autograd loss and gradients, and the layer program
+    ``compile_transformer`` lowers it to).  The inputs are stored next to the outputs, so the comparison does not depend on how
+    a machine's CPU kernels round."""
+    import dataclasses
+
+    from torch.nn.attention import SDPBackend, sdpa_kernel
+
+    from breaching.cases.models.language_models import TransformerModel
+
+    from breaching_b200 import compiler
+
+    case = dict(batch=2, seq_len=6, seed=77)
+    model, loss_fn, payload, shared, true = synthetic.make_text_case(**case)
+    cfg = refshim.load_reference_attack_cfg("tag", {})
+    att = ref.attacks.prepare_attack(model, loss_fn, cfg, dict(device=torch.device("cpu"), dtype=torch.float))
+    shared_in = [g.clone() for g in shared[0]["gradients"]]
+    sh_ref = copy.deepcopy(shared)
+    rec_models, _, _ = att.prepare_attack(payload, sh_ref)
+    dim = att.embeddings[0]["weight"].shape[1]
+    gen = torch.Generator().manual_seed(5)
+    rec_data = model.encoder.weight.detach()[true["data"]] + 0.01 * torch.randn(2, 6, dim, generator=gen)
+    recovered = {}
+    for mode in ("from-embedding", "from-labels", "from-limited-embedding"):
+        att.cfg.token_recovery = mode
+        recovered[mode] = att._postprocess_text_data(dict(data=rec_data.clone(), labels=true["data"].clone()))["data"]
+    text = dict(case=case, weight_checksum=float(sum(p.double().sum() for p in model.parameters())), text_strategy=cfg.text_strategy,
+                shared_gradients=shared_in, gradients_after=[g.clone() for g in sh_ref[0]["gradients"]],
+                embedding_weight=att.embeddings[0]["weight"].detach().clone(), embedding_grads=att.embeddings[0]["grads"].clone(),
+                dim=dim, data_shape=list(att.data_shape), param_names=[n for n, _ in rec_models[0].named_parameters()],
+                encoder_is_identity=isinstance(rec_models[0].encoder, torch.nn.Identity), rec_data=rec_data, tokens=true["data"].clone(),
+                recovered=recovered)
+
+    torch.manual_seed(4)
+    tm = TransformerModel(ntokens=40, ninp=16, nhead=4, nhid=24, nlayers=2, dropout=0.0, positional_embedding="learnable").eval()
+    weights = [p.detach().clone() for p in tm.parameters()]        # float32: .double() below converts them exactly
+    names = [n for n, _ in tm.named_parameters()]
+    tm = tm.double()
+    B, T = 2, 6
+    program = dataclasses.asdict(compiler.compile_transformer(tm, B, T, pad_vocab=False))
+    x = torch.randn(B, T, 16, dtype=torch.double, requires_grad=True)
+    q = torch.softmax(torch.randn(B, T, 40, dtype=torch.double), dim=-1)
+    tm.encoder = torch.nn.Identity()
+    with sdpa_kernel(SDPBackend.MATH):
+        loss = synthetic.causal_loss(tm(x), q)
+        grads = torch.autograd.grad(loss, list(tm.parameters()))
+    grads = [g.detach() for g in grads]
+    # a sequence of T positions reads the first T rows of the positional table: the other rows do not enter the loss and their
+    # gradient rows are exactly zero, so only the first T rows are kept
+    pos = names.index("pos_encoder.embedding.weight")
+    gpos = [n for n in names if n != "encoder.weight"].index("pos_encoder.embedding.weight")   # grads skip the token embedding
+    assert grads[gpos][T:].abs().max().item() == 0.0
+    weights[pos], grads[gpos] = weights[pos][:T].clone(), grads[gpos][:T].clone()
+    transformer = dict(ctor=dict(ntokens=40, ninp=16, nhead=4, nhid=24, nlayers=2), batch=B, seq_len=T, param_names=names, weights=weights,
+                       program=program, x=x.detach(), q=q, loss=float(loss), grads=grads)
+    return dict(text=text, transformer=transformer, torch_version=torch.__version__)
+
+
 def main():
+    sys.path.insert(0, os.path.dirname(HERE))
+    from helpers import FIXTURE_THREADS
+
+    torch.set_num_threads(FIXTURE_THREADS)   # the CPU replays in tests/ run with the same count
     ref = refshim.import_reference()
     torch.manual_seed(0)
     only = sys.argv[1:]   # optional: regenerate just the named fixtures
@@ -345,6 +408,8 @@ def main():
         torch.save(config_fixtures(), os.path.join(HERE, "attack_configs.pt"))
     if not only or "inits" in only:
         torch.save(init_fixtures(ref), os.path.join(HERE, "inits.pt"))
+    if not only or "dropin" in only:
+        torch.save(dropin_fixture(ref), os.path.join(HERE, "dropin.pt"))
     if only:
         return
     torch.save(label_fixtures(ref), os.path.join(HERE, "labels.pt"))

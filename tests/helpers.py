@@ -1,4 +1,5 @@
 """Shared helpers for the parity tests."""
+import contextlib
 import copy
 import os
 import sys
@@ -13,6 +14,22 @@ from breaching_b200 import config as bcfg  # noqa: E402
 from breaching_b200 import synthetic  # noqa: E402
 
 GOLDEN = os.path.join(ROOT, "tests", "golden")
+
+# The trajectory fixtures were generated with 8 intra-op CPU threads (tests/golden/make_golden.py).  CPU kernels split their
+# reductions by the thread count, and the FedAvg, train-mode BN and L-BFGS / joint trajectories amplify the resulting last-bit
+# differences past the tolerances of the CPU replays (FedAvg's first objective moves by 2e-4 relative below 8 threads), so
+# those replays run with the same count on any host.
+FIXTURE_THREADS = 8
+
+
+@contextlib.contextmanager
+def fixture_threads():
+    old = torch.get_num_threads()
+    torch.set_num_threads(FIXTURE_THREADS)
+    try:
+        yield
+    finally:
+        torch.set_num_threads(old)
 
 
 def load_golden(name):

@@ -5,8 +5,14 @@ import pytest
 import torch
 
 from helpers import (FEDAVG_FIXTURES, JOINT_FIXTURES, LBFGS_FIXTURES, MULTI_QUERY_FIXTURES, TRAIN_BN_FIXTURES, TRIAL_FIXTURES,
-                     joint_oracle_for_fixture,
+                     fixture_threads, joint_oracle_for_fixture,
                      load_golden, multi_query_oracle_for_fixture, oracle_for_fixture)
+
+
+@pytest.fixture(autouse=True)
+def _same_threads_as_the_fixtures():
+    with fixture_threads():
+        yield
 
 
 @pytest.mark.parametrize("name", TRIAL_FIXTURES + FEDAVG_FIXTURES + LBFGS_FIXTURES + TRAIN_BN_FIXTURES)
