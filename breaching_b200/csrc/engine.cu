@@ -384,10 +384,14 @@ struct bre_engine {
     }
     return mask;
   }
+  // gemm_on's choice of the tcgen05 kernel (the only one that applies an epilogue)
+  bool runs_on_tc(const GemmArgs& a) const {
+    return !linear_tall_supported(a) && !linear_small_preferred(a) && gemm_backend == 1 && !a.force_fp32 && igemm_tc_supported(a);
+  }
   int gemm_on(const GemmArgs& a, cudaStream_t st) {
     if (linear_tall_supported(a)) return launch_linear_tall(a, st);
     if (linear_small_preferred(a)) return launch_linear_small(a, st);
-    if (gemm_backend == 1 && !a.force_fp32 && igemm_tc_supported(a)) {
+    if (runs_on_tc(a)) {
       GemmArgs b = a;
       b.wgt_static = static_weights(a);
       return launch_igemm_tc(b, st);
@@ -395,11 +399,12 @@ struct bre_engine {
     return launch_igemm_simt(a, st);
   }
 
-  // The BN/residual/ReLU op that directly follows conv `i` and reads its output can run in the GEMM epilogue (tcgen05 back end).
+  // The BN/residual/ReLU op that directly follows conv `i` and reads its output can run in the GEMM epilogue, when the GEMM runs
+  // on the tcgen05 kernel (a precise layer runs on the fp32 kernel, which has no epilogue).
   bool fuses_with_next(size_t i, const GemmArgs& a) const {
-    if (!fuse_bnact || gemm_backend != 1 || i + 1 >= ops.size()) return false;
+    if (!fuse_bnact || i + 1 >= ops.size()) return false;
     const bre_op_desc& nx = ops[i + 1];
-    return nx.kind == BRE_OP_BNACT && nx.tin == ops[i].tout && !nx.bn_train && igemm_tc_supported(a);
+    return nx.kind == BRE_OP_BNACT && nx.tin == ops[i].tout && !nx.bn_train && runs_on_tc(a);
   }
   int consumers_of(int tensor) const {
     int n = 0;
@@ -645,7 +650,8 @@ struct bre_engine {
             a.epi.scale = c.scale; a.epi.inv = c.inv; a.epi.nrm = c.nrm;
             a.epi.v_gamma = nx.has_bn ? Vp(nx.gamma) : nullptr; a.epi.v_beta = nx.has_bn ? Vp(nx.beta) : nullptr;
             a.epi.pre = t[nx.tin].val; a.epi.post = t[nx.tout].val;
-            if (consumers_of(op.tout) == 1) a.out = nullptr;   // nobody else reads the pre-BN tangent
+            // nobody else reads the pre-BN tangent, unless the tangent gamma-gradient of a FedAvg step does (sweep_tangent_backward)
+            if (consumers_of(op.tout) == 1 && !want_tangent_G) a.out = nullptr;
             ++i;
           }
           BRE_LAUNCH(gemm(a));

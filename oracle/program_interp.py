@@ -399,6 +399,7 @@ class ProgramInterpreter:
             centred = (zdot - (p * zdot).sum(dim=1, keepdim=True)) * self.row_keep
             seed = p * centred / self.M
             d, _, _ = self._reverse(seed, V=V, d_prev=self.d_B, inject=inject)
+            self.d_TB = d
             # d objective / d (target probabilities): row (b, t) receives the term of the logits row (b, t - 1)
             dq = torch.zeros_like(centred)
             dq[1:] = -centred[:-1] / self.M
@@ -406,6 +407,7 @@ class ProgramInterpreter:
             return d[0].flatten(1).view(n // T, T, -1)
         seed = (p * zdot - p * (p * zdot).sum(dim=1, keepdim=True)) / n
         d, _, _ = self._reverse(seed, V=V, d_prev=self.d_B, inject=inject)
+        self.d_TB = d
         return d[0]
 
     # ------------------------------------------------------------------ regulariser adjoints

@@ -32,6 +32,69 @@ def fixture_threads():
         torch.set_num_threads(old)
 
 
+class OddChannelNet(torch.nn.Module):
+    """3 -> 6 -> 10 -> 14 channels (none a multiple of 4: the scalar element-wise kernels), a residual add onto a tensor that also
+    feeds a convolution (accumulated deltas), 3/2/1 max-pooling after a ReLU on a 15 x 13 map, average pooling, 7 classes."""
+
+    def __init__(self, classes=7):
+        super().__init__()
+        nn = torch.nn
+        self.conv0, self.bn0 = nn.Conv2d(3, 6, 3, padding=1), nn.BatchNorm2d(6)
+        self.conv1, self.bn1 = nn.Conv2d(6, 10, 3, padding=1, bias=False), nn.BatchNorm2d(10)
+        self.conv2, self.bn2 = nn.Conv2d(10, 10, 3, padding=1, bias=False), nn.BatchNorm2d(10)
+        self.pool = nn.MaxPool2d(3, 2, 1)
+        self.conv3, self.bn3 = nn.Conv2d(10, 14, 3, padding=1), nn.BatchNorm2d(14)
+        self.avg = nn.AdaptiveAvgPool2d(1)
+        self.fc = nn.Linear(14, classes)
+
+    def forward(self, x):
+        h = torch.relu(self.bn0(self.conv0(x)))
+        h1 = torch.relu(self.bn1(self.conv1(h)))
+        h2 = torch.relu(self.bn2(self.conv2(h1)) + h1)
+        h3 = torch.relu(self.bn3(self.conv3(self.pool(h2))))
+        return self.fc(torch.flatten(self.avg(h3), 1))
+
+
+class TensorCoreNet(torch.nn.Module):
+    """Channel counts the tcgen05 kernels take with both tile widths: a 3-channel stem, 32 -> 96 and 96 -> 64 layers (128 x 32
+    tiles), 64-channel layers (128 x 64 tiles), a stride-2 3 x 3 convolution and a 1 x 1 stride-2 downsample added back."""
+
+    def __init__(self, classes=10):
+        super().__init__()
+        nn = torch.nn
+        self.stem, self.bn0 = nn.Conv2d(3, 32, 3, padding=1, bias=False), nn.BatchNorm2d(32)
+        self.conv1, self.bn1 = nn.Conv2d(32, 96, 3, padding=1, bias=False), nn.BatchNorm2d(96)
+        self.conv2, self.bn2 = nn.Conv2d(96, 64, 3, padding=1, bias=False), nn.BatchNorm2d(64)
+        self.conv3, self.bn3 = nn.Conv2d(64, 64, 3, stride=2, padding=1, bias=False), nn.BatchNorm2d(64)
+        self.conv4, self.bn4 = nn.Conv2d(64, 64, 3, padding=1, bias=False), nn.BatchNorm2d(64)
+        self.down, self.bnd = nn.Conv2d(64, 64, 1, stride=2, bias=False), nn.BatchNorm2d(64)
+        self.avg = nn.AdaptiveAvgPool2d(1)
+        self.fc = nn.Linear(64, classes)
+
+    def forward(self, x):
+        h = torch.relu(self.bn0(self.stem(x)))
+        h = torch.relu(self.bn1(self.conv1(h)))
+        h = torch.relu(self.bn2(self.conv2(h)))
+        y = torch.relu(self.bn3(self.conv3(h)))
+        y = torch.relu(self.bn4(self.conv4(y)) + self.bnd(self.down(h)))
+        return self.fc(torch.flatten(self.avg(y), 1))
+
+
+def parity_model(name, seed=0, train_bn=False):
+    """``odd`` / ``tensor-core``: randomly initialised, BN with random affine parameters and running statistics (eval mode), or
+    train-mode BN without running statistics (``train_bn``)."""
+    torch.manual_seed(seed)
+    model = OddChannelNet() if name == "odd" else TensorCoreNet()
+    synthetic.randomize_bn(model, seed + 1)
+    model.eval()
+    if train_bn:
+        model.train()
+        for mod in model.modules():
+            if isinstance(mod, torch.nn.BatchNorm2d):
+                mod.track_running_stats = False
+    return model
+
+
 def load_golden(name):
     return torch.load(os.path.join(GOLDEN, name), weights_only=False)
 

@@ -132,18 +132,34 @@ def test_total_variation_value_and_gradient(p, q, dbl, shape):
     assert _relerr(acc.cpu(), 2 * gref) < 5e-5
 
 
-TC_SHAPES = [s for s in CONV_SHAPES if s[3] % 32 == 0 and s[4] % 64 == 0] + [
+def tc_claims(mode, shape):
+    """Does the tcgen05 back end take this NHWC convolution (igemm_tc_supported / narrow_tiles_ok)?  Output tiles are 128 x 64, or
+    128 x 32 where the tile width (fprop: Co, dgrad: Ci, wgrad: R R Ci) is only a multiple of 32 -- and then dgrad only at stride 1,
+    wgrad only with Ci % 32 == 0."""
+    N, H, W, Ci, Co, R, st, pd = shape
+    width = {0: Co, 1: Ci, 2: R * R * Ci}[mode]
+    narrow_ok = (mode != 1 or st == 1) and (mode != 2 or Ci % 32 == 0)
+    if R * R > 64 or not (width % 64 == 0 or (width % 32 == 0 and narrow_ok)):
+        return False
+    return {0: Ci % 32 == 0, 1: Co % 32 == 0, 2: Co % 4 == 0 and Ci % 4 == 0}[mode]
+
+
+TC_SHAPES = [s for s in CONV_SHAPES if tc_claims(0, s)] + [
     (1, 56, 56, 64, 64, 3, 1, 1), (8, 14, 14, 128, 256, 3, 2, 1),
     (1, 2, 2, 512, 512, 3, 1, 1), (1, 4, 4, 256, 256, 3, 1, 1), (4, 8, 8, 128, 128, 3, 1, 1),   # tiny spatial extents (64x64 inputs)
     (3, 9, 11, 64, 64, 3, 1, 1), (2, 15, 13, 64, 128, 3, 2, 1), (1, 5, 5, 96, 64, 3, 1, 1),    # ragged tiles, odd sizes, Ci = 96
     (8, 56, 56, 64, 256, 1, 1, 0), (8, 28, 28, 128, 128, 3, 1, 1), (2, 28, 28, 256, 64, 1, 2, 0),  # ResNet-50 batch-8 shapes
+    # 128 x 32 tiles: Co / Ci in {32, 96}, stride 1 and 2, 1 x 1 and 3 x 3, ragged spatial sizes
+    (2, 33, 29, 32, 96, 3, 1, 1), (2, 33, 29, 96, 64, 3, 1, 1), (2, 15, 13, 32, 32, 3, 1, 1), (3, 9, 11, 96, 96, 1, 1, 0),
+    (2, 15, 13, 96, 32, 3, 2, 1), (2, 17, 11, 32, 96, 1, 2, 0), (1, 7, 9, 64, 32, 3, 1, 1), (2, 13, 15, 32, 64, 3, 2, 1),
 ]
 
 
 @pytest.mark.parametrize("shape", TC_SHAPES)
 def test_conv_tcgen05_tf32_backend(shape):
     """tcgen05 TF32 back end (tensor cores, TMEM accumulators): TF32 products (10-bit mantissa), fp32 accumulation,
-    tolerance 2e-3 relative l2 -- the precision of the reference's default cuDNN TF32 conv path."""
+    tolerance 2e-3 relative l2 -- the precision of the reference's default cuDNN TF32 conv path.  Every mode the dispatcher
+    claims must be accepted (a refusal raises), every other mode refused."""
     N, H, W, Ci, Co, R, st, pd = shape
     x = _rand(N, Ci, H, W, seed=1)
     w = _rand(Co, Ci, R, R, seed=2) * 0.1
@@ -159,13 +175,19 @@ def test_conv_tcgen05_tf32_backend(shape):
     again = torch.empty_like(out)
     E.conv_gemm(0, _nhwc(x), w_ohwi, again, N, H, W, Ci, Co, R, R, st, pd, a2=_nhwc(x2), w2=w2_ohwi, backend=1)
     assert torch.equal(out, again)
-    if Ci % 64 == 0:
+    assert tc_claims(0, shape)
+    for mode in (1, 2):
+        if not tc_claims(mode, shape):
+            with pytest.raises(E.EngineError):
+                E.conv_gemm(mode, _nhwc(dy) if mode == 1 else _nhwc(x), w_ohwi if mode == 1 else _nhwc(dy),
+                            torch.empty(N * H * W * Ci if mode == 1 else Co * R * R * Ci, device=DEV), N, H, W, Ci, Co, R, R, st, pd, backend=1)
+    if tc_claims(1, shape):
         din = torch.empty(N, H, W, Ci, device=DEV)
         E.conv_gemm(1, _nhwc(dy), w_ohwi, din, N, H, W, Ci, Co, R, R, st, pd, a2=_nhwc(dy2), w2=w2_ohwi, backend=1)
         refd = torch.nn.grad.conv2d_input((N, Ci, H, W), w.double(), dy.double(), stride=st, padding=pd) + \
             torch.nn.grad.conv2d_input((N, Ci, H, W), w2.double(), dy2.double(), stride=st, padding=pd)
         assert _relerr(din.permute(0, 3, 1, 2), refd) < tol, "dgrad dual"
-    if (R * R * Ci) % 64 == 0:
+    if tc_claims(2, shape):
         dw = torch.empty(Co, R, R, Ci, device=DEV)
         E.conv_gemm(2, _nhwc(x), _nhwc(dy), dw, N, H, W, Ci, Co, R, R, st, pd, backend=1)
         refw = torch.nn.grad.conv2d_weight(x.double(), (Co, Ci, R, R), dy.double(), stride=st, padding=pd)

@@ -5,18 +5,29 @@ import torch
 from breaching_b200 import compiler, config, synthetic
 from oracle import program_interp as PI
 from oracle import restate
+from helpers import parity_model
 
 KINDS = ["cosine-similarity", "euclidean", "l1", "tag-euclidean", "angular", "fast-cosine-similarity",
          "masked-cosine-similarity"]
 
 
 def _setup(mname, data, size, batch, kind, treg=0.0, regs=None):
-    model, loss_fn, payload, shared, true = synthetic.make_case(mname, data, batch=batch, seed=3, bn_random=True,
-                                                                image_size=size, classes=10)
+    H, W = (size, size) if isinstance(size, int) else size
+    if mname in ("odd", "tensor-core"):   # the test models of tests/test_sweep_tensors_gpu.py, at their ragged sizes
+        model = parity_model(mname, seed=3)
+        gen = torch.Generator().manual_seed(4)
+        xt = torch.randn(batch, 3, H, W, generator=gen)
+        labels = torch.randint(0, model.fc.out_features, (batch,), generator=gen)
+        loss_fn = torch.nn.CrossEntropyLoss()
+        grads = torch.autograd.grad(loss_fn(model(xt), labels), list(model.parameters()))
+        shared, true = [dict(gradients=grads)], dict(labels=labels)
+    else:
+        model, loss_fn, payload, shared, true = synthetic.make_case(mname, data, batch=batch, seed=3, bn_random=True,
+                                                                    image_size=size, classes=10)
     model = model.double().eval()
     g = [t.double() for t in shared[0]["gradients"]]
     gen = torch.Generator().manual_seed(5)
-    x = torch.randn(batch, 3, size, size, dtype=torch.double, generator=gen)
+    x = torch.randn(batch, 3, H, W, dtype=torch.double, generator=gen)
     cfg = config.get_attack_config("invertinggradients", {"objective.type": kind, "objective.task_regularization": treg,
                                                            "regularization": regs})
     dm, ds = torch.zeros(1, 3, 1, 1), torch.ones(1, 3, 1, 1)
@@ -25,7 +36,8 @@ def _setup(mname, data, size, batch, kind, treg=0.0, regs=None):
 
 
 @pytest.mark.parametrize("kind", KINDS)
-@pytest.mark.parametrize("mname,data,size", [("convnet-tiny", "cifar", 32), ("resnet18", "imagenet", 32)])
+@pytest.mark.parametrize("mname,data,size", [("convnet-tiny", "cifar", 32), ("resnet18", "imagenet", 32), ("odd", None, (15, 13)),
+                                             ("tensor-core", None, (33, 29))])
 def test_tangent_formulation_matches_double_backward(mname, data, size, kind):
     model, g, x, labels, cfg, orc = _setup(mname, data, size, 2, kind, treg=0.3)
     phi, _, raw, _ = orc.closure_gradient(x, 0, 0.1)
